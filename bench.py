@@ -8,7 +8,7 @@ every factor (residual + Jacobian) -> loss reweighting -> J^T J / J^T r -> landm
 `value` = factors per second with everything resident in HBM; `e2e` = the same through
 hb200_optimize() with the variable blocks in pinned HOST memory (H2D + D2H inside the timed region).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1] [--impl reference] [--dump-outputs DIR]
 N > 1: launched by torch.distributed.run, one rank per GPU, weak scaling on the headline workload (each rank
 owns one cfg-sized factor shard of an N-times larger window) plus strong-scaling sections on the large
 BASELINE configs (cfg3: 500 k pixel factors, cfg4: 1 M factors) sharded over the N ranks.
@@ -46,6 +46,7 @@ def parse_args():
     p.add_argument("--no-large", action="store_true", help="skip the large-window sections (cfg2 / cfg3 / cfg4)")
     p.add_argument("--no-parity", action="store_true", help="skip the N-rank vs oracle check at N > 1")
     p.add_argument("--sweep", action="store_true", help="factor-count sweep of the 1 M-factor window (BASELINE config 5)")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64, single GPU)")
     return p.parse_args()
 
 
@@ -273,6 +274,17 @@ class Harness:
         self.ctx.close()
 
 
+def dump_outputs(out_dir, ctx):
+    """What a caller of the timed step receives: the window state after the last timed LM iteration, and the pose /
+    landmark step that iteration solved for.  The window is seeded, so two builds can be compared array by array, to
+    rounding (DESIGN.md section 6); the largest config, cfg4, writes about 4 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = ctx.state()
+    arrays["delta_p"], arrays["delta_l"] = ctx.delta()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def roofline_entry(name, nbytes, ms, peak):
     ach = nbytes / (ms * 1e-3) / 1e9
     return dict(kernel=name, algorithmic_bytes_per_launch=int(nbytes), launch_ms=ms, achieved=ach, frac=ach / peak)
@@ -397,6 +409,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (world > 1 or args.impl != "b200"):
+        raise SystemExit("--dump-outputs covers --impl b200 on one GPU (at N > 1 a rank's landmarks are only its own shard's)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -431,6 +445,8 @@ def main():
     ms_per_step = total_ms / args.steps
     value = nf_total / (ms_per_step * 1e-3)
     info = ctx.comm_info()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ctx)   # before the evaluate sweep below restores the snapshot
 
     # evaluate-only sweep (knot table + factor kernels, residual + Jacobian)
     sweep_ms, _ = h.timed_steps(lambda: ctx.evaluate(jacobians=True), args.steps, 3)
