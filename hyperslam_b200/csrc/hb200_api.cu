@@ -423,14 +423,18 @@ int ensure_system(hb200_ctx* c) {
   if (c->band_solver && !c->use_bcr) {
     if (c->band_smem) HB_CUDA(cudaFuncSetAttribute(band_solve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ws)));
     else {
-      HB_CUDA(c->band_ws.ensure(ws / sizeof(double)));
       // chunked factorisation: two shared-memory views of band_chunk_cols block columns (band + arrow + LI)
       const size_t colbytes = (static_cast<size_t>(6 + 6 * c->beta) * 6 + 6 * static_cast<size_t>(c->n - 6 * c->K + 1) + 48) * sizeof(double);
       const int fit = static_cast<int>((200 * 1024) / (2 * colbytes));
       c->band_chunk_cols = std::max(c->beta + 2, std::min(fit, c->K + c->beta));
       c->band_chunk_smem = 2 * colbytes * c->band_chunk_cols;
-      if (c->band_chunk_smem > 220 * 1024) return fail(-6, "band solver: a chunk of %d block columns does not fit shared memory (arrow too wide)", c->band_chunk_cols);
-      HB_CUDA(cudaFuncSetAttribute(band_solve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->band_chunk_smem)));
+      // the chunk needs beta + 2 block columns: a wide band (landmark tracks of 17+ control points) or a wide arrow
+      // leaves no band plan, and the dense cooperative Cholesky solves the window instead
+      if (c->band_chunk_smem > 220 * 1024) c->band_solver = false;
+      else {
+        HB_CUDA(c->band_ws.ensure(ws / sizeof(double)));
+        HB_CUDA(cudaFuncSetAttribute(band_solve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->band_chunk_smem)));
+      }
     }
   }
   HB_CUDA(c->band_ws.ensure(1));
@@ -616,7 +620,7 @@ int enqueue_build(hb200_ctx* c, bool pixel_fused = false) {
       else HB_IMU_MMA(6, 12);
 #undef HB_IMU_MMA
     }
-    HB_LAUNCH(c, "inertial_hessian_kernel");
+    HB_LAUNCH(c, scalar_hess ? "inertial_hessian_kernel" : "inertial_hessian_mma_kernel");
   }
   if (c->Nm) {
     const int blocks = (c->Nm + kManWarps - 1) / kManWarps;
@@ -683,7 +687,7 @@ int enqueue_solve(hb200_ctx* c, bool fuse_retract = false, bool* fused = nullptr
     const size_t smem = c->band_smem ? band_workspace_doubles(c->K, c->beta, c->n - 6 * c->K) * sizeof(double) : 0;
     if (c->band_smem) band_solve_kernel<true><<<1, kBandThreads, smem, c->stream>>>(c->sys.p, c->lay, c->band_ws.p, c->dp.p, c->spd.p, c->band_dbg.p, st, fx, Dout, 0);
     else band_solve_kernel<false><<<1, kBandThreads, c->band_chunk_smem, c->stream>>>(c->sys.p, c->lay, c->band_ws.p, c->dp.p, c->spd.p, c->band_dbg.p, st, fx, Dout, c->band_chunk_cols);
-    HB_LAUNCH(c, "band_solve_kernel");
+    HB_LAUNCH(c, c->band_smem ? "band_solve_kernel" : "band_solve_kernel<chunked>");
   } else {
     { const int rd = enqueue_densify(c); if (rd) return rd; }
     int n = c->n;

@@ -3,13 +3,14 @@
   cfg3  4-camera rig, 500 knots, 500 k pixel factors       (n = 3 026)
   cfg4  1 M factors (833 k pixel + 167 k IMU), 500 knots    (n = 3 026)
 Every factor's index map, residual and Jacobian, the full reduced system, the LM step and three LM iterations
-are compared with the CPU oracle on the same seeded window -- the chunked (out-of-shared-memory) band solver is the
-default path at these sizes; cfg2 is repeated with the dense cooperative Cholesky.
+are compared with the CPU oracle on the same seeded window (the reduced system block by block, tests/system_blocks.py)
+-- the chunked (out-of-shared-memory) band solver is the default path at these sizes; cfg2 is repeated with the dense cooperative Cholesky.
 """
 import numpy as np
 import pytest
 
 import oracle_lib as ol
+import system_blocks as sb
 from hyperslam_b200 import runtime, synthetic
 
 pytestmark = pytest.mark.gpu
@@ -54,8 +55,7 @@ def test_full_size_config_parity(built, config, force_dense):
     o = ow.iterate(apply=False)
     ctx.build_system()
     S, b = ctx.system()
-    assert rel_err(S, o["S"]) < 1e-9
-    assert rel_err(b, o["b"]) < 1e-9
+    sb.assert_system_close(S, b, o["S"], o["b"], sb.DofLayout.of(win))
     ctx.solve()
     dp, dl = ctx.delta()
     res = np.abs(o["S"] @ dp - o["b"]).max() / (np.abs(o["b"]).max() + 1e-300)
