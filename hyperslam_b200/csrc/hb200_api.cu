@@ -218,9 +218,10 @@ struct hb200_ctx {
   // device-side window bookkeeping (hb200_append_* / hb200_slide): the factor lists live on the device only, the host
   // mirrors above are refreshed on demand (sync_host_mirrors)
   bool device_managed = false;
-  DevBuf<double> alt_stamp, alt_meas, alt_lms, alt_knots;
+  DevBuf<double> alt_stamp, alt_meas, alt_lms, alt_knots, alt_z;
   DevBuf<double2> alt_pixel;
   DevBuf<int4> alt_idx;
+  DevBuf<int2> alt_midx;
   DevBuf<int> w_keep, w_pos, w_lkeep, w_lpos, w_cnt, w_scal;
   DevBuf<unsigned long long> w_last;
   // outputs
@@ -1212,17 +1213,21 @@ int hb200_set_inertial_factors(hb200_ctx* c, int n, const double* stamp, const d
 }  // extern "C"
 
 namespace {
-// After hb200_append_* / hb200_slide the factor lists exist on the device only (bound order == user order from
-// then on).  The host mirrors the copy-out calls and a later full hb200_bind need are refreshed here, on demand.
+// After hb200_append_* / hb200_slide the factor lists exist on the device only (bound order == list order from then
+// on).  The host mirrors the copy-out calls and a later full hb200_bind need are refreshed here, on demand.  The visual
+// list splits by kind (idx.w): the pixel factors keep their list order as user order, a bearing factor's user index is
+// Np + its rank among the bearings; the manifold list is in user order as it stands.
 int sync_host_mirrors(hb200_ctx* c) {
   if (!c->device_managed) return 0;
   HB_CUDA(cudaSetDevice(c->device));
-  const size_t Nv = c->Nv, Ni = c->Ni;
-  c->h_p_stamp.resize(Nv); c->h_p_pixel.resize(2 * Nv); c->h_p_cam.resize(Nv); c->h_p_lm.resize(Nv);
+  const size_t Nv = c->Nv, Ni = c->Ni, Nm = c->Nm;
+  std::vector<double> st(Nv), px(2 * Nv), vz(Nv);
   c->h_v_idx.resize(Nv); c->h_i_idx.resize(Ni); c->h_i_stamp.resize(Ni); c->h_i_meas.resize(6 * Ni);
+  c->h_m_idx.resize(Nm); c->h_m_stamp.resize(Nm); c->h_m_meas.resize(7 * Nm);
   if (Nv) {
-    HB_CUDA(cudaMemcpyAsync(c->h_p_stamp.data(), c->v_stamp.p, sizeof(double) * Nv, cudaMemcpyDeviceToHost, c->stream));
-    HB_CUDA(cudaMemcpyAsync(c->h_p_pixel.data(), c->v_pixel.p, sizeof(double) * 2 * Nv, cudaMemcpyDeviceToHost, c->stream));
+    HB_CUDA(cudaMemcpyAsync(st.data(), c->v_stamp.p, sizeof(double) * Nv, cudaMemcpyDeviceToHost, c->stream));
+    HB_CUDA(cudaMemcpyAsync(px.data(), c->v_pixel.p, sizeof(double) * 2 * Nv, cudaMemcpyDeviceToHost, c->stream));
+    HB_CUDA(cudaMemcpyAsync(vz.data(), c->v_z.p, sizeof(double) * Nv, cudaMemcpyDeviceToHost, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->h_v_idx.data(), c->v_idx.p, sizeof(int4) * Nv, cudaMemcpyDeviceToHost, c->stream));
   }
   if (Ni) {
@@ -1230,12 +1235,38 @@ int sync_host_mirrors(hb200_ctx* c) {
     HB_CUDA(cudaMemcpyAsync(c->h_i_meas.data(), c->i_meas.p, sizeof(double) * 6 * Ni, cudaMemcpyDeviceToHost, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->h_i_idx.data(), c->i_idx.p, sizeof(int4) * Ni, cudaMemcpyDeviceToHost, c->stream));
   }
+  if (Nm) {
+    HB_CUDA(cudaMemcpyAsync(c->h_m_stamp.data(), c->m_stamp.p, sizeof(double) * Nm, cudaMemcpyDeviceToHost, c->stream));
+    HB_CUDA(cudaMemcpyAsync(c->h_m_meas.data(), c->m_meas.p, sizeof(double) * 7 * Nm, cudaMemcpyDeviceToHost, c->stream));
+    HB_CUDA(cudaMemcpyAsync(c->h_m_idx.data(), c->m_idx.p, sizeof(int2) * Nm, cudaMemcpyDeviceToHost, c->stream));
+  }
   HB_CUDA(cudaStreamSynchronize(c->stream));
-  for (size_t f = 0; f < Nv; ++f) { c->h_p_cam[f] = c->h_v_idx[f].z; c->h_p_lm[f] = c->h_v_idx[f].y; }
-  c->h_v_stamp = c->h_p_stamp; c->h_v_pixel = c->h_p_pixel; c->h_v_cam = c->h_p_cam; c->h_v_lm = c->h_p_lm; c->h_v_z.assign(Nv, 0.0);
-  c->v_perm.resize(Nv); std::iota(c->v_perm.begin(), c->v_perm.end(), 0);
+  c->h_p_stamp.clear(); c->h_p_pixel.clear(); c->h_p_cam.clear(); c->h_p_lm.clear();
+  c->h_b_stamp.clear(); c->h_b_bearing.clear(); c->h_b_cam.clear(); c->h_b_lm.clear();
+  for (size_t f = 0; f < Nv; ++f) {
+    const int4 id = c->h_v_idx[f];
+    if (id.w == 0) {
+      c->h_p_stamp.push_back(st[f]); c->h_p_pixel.push_back(px[2 * f]); c->h_p_pixel.push_back(px[2 * f + 1]);
+      c->h_p_cam.push_back(id.z); c->h_p_lm.push_back(id.y);
+    } else {
+      c->h_b_stamp.push_back(st[f]); c->h_b_bearing.push_back(px[2 * f]); c->h_b_bearing.push_back(px[2 * f + 1]); c->h_b_bearing.push_back(vz[f]);
+      c->h_b_cam.push_back(id.z); c->h_b_lm.push_back(id.y);
+    }
+  }
+  c->Np = static_cast<int>(c->h_p_stamp.size()); c->Nb = static_cast<int>(c->h_b_stamp.size());
+  // user-order visual list (pixel factors, then bearing factors: what rebuild_visual assembles) and bound position -> user index
+  c->h_v_stamp.resize(Nv); c->h_v_pixel.resize(2 * Nv); c->h_v_z.assign(Nv, 0.0); c->h_v_cam.resize(Nv); c->h_v_lm.resize(Nv);
+  c->v_perm.resize(Nv);
+  for (size_t f = 0, ip = 0, ib = 0; f < Nv; ++f) {
+    const size_t u = (c->h_v_idx[f].w == 0) ? ip++ : c->Np + ib++;
+    c->v_perm[f] = static_cast<int>(u);
+    c->h_v_stamp[u] = st[f]; c->h_v_pixel[2 * u] = px[2 * f]; c->h_v_pixel[2 * u + 1] = px[2 * f + 1];
+    c->h_v_cam[u] = c->h_v_idx[f].z; c->h_v_lm[u] = c->h_v_idx[f].y;
+    if (c->h_v_idx[f].w) c->h_v_z[u] = vz[f];
+  }
+  c->h_m_sensor.resize(Nm);
+  for (size_t f = 0; f < Nm; ++f) c->h_m_sensor[f] = c->h_m_idx[f].y;
   c->i_perm.resize(Ni); std::iota(c->i_perm.begin(), c->i_perm.end(), 0);
-  c->Np = static_cast<int>(Nv);
   c->device_managed = false;
   return 0;
 }
@@ -1243,7 +1274,7 @@ int sync_host_mirrors(hb200_ctx* c) {
 // Incidence lists of the device-resident factor lists (landmark CSR, inertial runs, segment offsets, longest
 // track) by counting + scan kernels, then everything hb200_bind derives from them.  One small read-back.
 int rebuild_incidence_device(hb200_ctx* c) {
-  const int Nv = c->Nv, Ni = c->Ni, L = c->L, K = c->K;
+  const int Nv = c->Nv, Ni = c->Ni, Nm = c->Nm, L = c->L, K = c->K;
   c->nseg = K - c->k + 1;
   HB_CUDA(c->w_scal.ensure(8));
   HB_CUDA(cudaMemsetAsync(c->w_scal.p, 0, 8 * sizeof(int), c->stream));
@@ -1286,14 +1317,15 @@ int rebuild_incidence_device(hb200_ctx* c) {
   if (2 * 3 * static_cast<size_t>(c->max_rows) * sizeof(double) > 200 * 1024) return fail(-6, "landmark track spans %d control-point dofs; exceeds the Schur kernel's shared-memory tile", c->max_rows);
   // outputs and launch shapes (as hb200_bind)
   const size_t k = c->k;
-  HB_CUDA(c->v_z.ensure(std::max(Nv, 1))); HB_CUDA(c->v_w.ensure(std::max(Nv, 1)));
+  HB_CUDA(c->v_z.grow(std::max(Nv, 1), Nv, c->stream)); HB_CUDA(c->v_w.ensure(std::max(Nv, 1)));   // (v_z holds the bearings' third components)
   HB_CUDA(c->v_r.ensure(2 * static_cast<size_t>(std::max(Nv, 1)))); HB_CUDA(c->v_Jp.ensure(12 * k * std::max(Nv, 1))); HB_CUDA(c->v_Jl.ensure(6 * static_cast<size_t>(std::max(Nv, 1))));
   HB_CUDA(c->i_r.ensure(6 * static_cast<size_t>(std::max(Ni, 1)))); HB_CUDA(c->i_Jp.ensure(36 * k * std::max(Ni, 1)));
   HB_CUDA(c->i_wg.ensure(4 * static_cast<size_t>(std::max(Ni, 1)))); HB_CUDA(c->i_wa.ensure(4 * static_cast<size_t>(std::max(Ni, 1)))); HB_CUDA(c->i_Jg.ensure(12 * static_cast<size_t>(std::max(Ni, 1))));
   c->n_pix_blocks = (Nv + kEvalThreads - 1) / kEvalThreads;
   c->n_imu_blocks = (Ni + kEvalThreads - 1) / kEvalThreads;
-  c->n_man_blocks = 0;
-  for (int s2 = 0; s2 < 2; ++s2) { HB_CUDA(c->cp_pix[s2].ensure(std::max(c->n_pix_blocks, 1))); HB_CUDA(c->cp_imu[s2].ensure(std::max(c->n_imu_blocks, 1))); }
+  c->n_man_blocks = (Nm + kEvalThreads - 1) / kEvalThreads;
+  HB_CUDA(c->m_r.ensure(6 * static_cast<size_t>(std::max(Nm, 1)))); HB_CUDA(c->m_Jp.ensure(36 * k * std::max(Nm, 1)));
+  for (int s2 = 0; s2 < 2; ++s2) { HB_CUDA(c->cp_pix[s2].ensure(std::max(c->n_pix_blocks, 1))); HB_CUDA(c->cp_imu[s2].ensure(std::max(c->n_imu_blocks + c->n_man_blocks, 1))); }
   if (c->max_rows * 6 * sizeof(double) > 48 * 1024) {
     const int smem = static_cast<int>(2 * 3 * static_cast<size_t>(c->max_rows) * sizeof(double));
     HB_CUDA(cudaFuncSetAttribute(schur_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -1337,7 +1369,7 @@ int hb200_bind(hb200_ctx* c, int* num_invalid) {
     HB_CUDA(cudaMemcpyAsync(c->v_stamp.p, c->h_v_stamp.data(), sizeof(double) * Nv, cudaMemcpyHostToDevice, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->v_cam.p, c->h_v_cam.data(), sizeof(int) * Nv, cudaMemcpyHostToDevice, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->v_lm.p, c->h_v_lm.data(), sizeof(int) * Nv, cudaMemcpyHostToDevice, c->stream));
-    bind_pixel_kernel<<<(Nv + 127) / 128, 128, 0, c->stream>>>(Nv, c->v_stamp.p, c->v_cam.p, c->v_lm.p, c->knots[0].p, c->K, c->k, c->C, c->L, c->v_idx.p, c->d_invalid.p);
+    bind_pixel_kernel<<<(Nv + 127) / 128, 128, 0, c->stream>>>(Nv, c->v_stamp.p, c->v_cam.p, c->v_lm.p, c->knots[0].p, c->K, c->k, c->C, c->L, 0, c->v_idx.p, c->d_invalid.p);
     HB_LAUNCH(c, "bind_pixel_kernel");
     HB_CUDA(cudaMemcpyAsync(c->h_v_idx.data(), c->v_idx.p, sizeof(int4) * Nv, cudaMemcpyDeviceToHost, c->stream));
   }
@@ -1539,6 +1571,7 @@ int hb200_get_pixel_outputs(hb200_ctx* c, double* r, double* Jp, double* Jl) {
 
 int hb200_get_bearing_outputs(hb200_ctx* c, double* r, double* Jp, double* Jl) {
   if (!c || !c->bound) return fail(-2, "not bound");
+  { const int rs = sync_host_mirrors(c); if (rs) return rs; }
   HB_CUDA(cudaSetDevice(c->device));
   const size_t N = c->Nv, w = 12 * static_cast<size_t>(c->k);
   if (c->Nb == 0) return 0;
@@ -2243,7 +2276,27 @@ namespace {
 int check_device_window(hb200_ctx* c) {
   if (!c) return fail(-1, "null context");
   if (!c->bound) return fail(-2, "bind the window first (hb200_bind)");
-  if (c->Nb || c->Nm) return fail(-4, "device-side window bookkeeping covers pixel and inertial factors (bearing / manifold lists must be empty)");
+  return 0;
+}
+
+// the visual list's tail [Nv, Nv + n) after a bind on the device: kind check of the stamps / indices (rc 2), then the
+// arrival order (rc 3).  The caller commits the new size only when both pass, so a rejected append changes nothing.
+int check_visual_tail(hb200_ctx* c, int Nv, int n) {
+  tail_sorted_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(Nv, n, c->v_idx.p, c->d_invalid.p + 1);
+  HB_LAUNCH(c, "tail_sorted_kernel");
+  int bad[2] = {0, 0};
+  HB_CUDA(cudaMemcpyAsync(bad, c->d_invalid.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  HB_CUDA(cudaStreamSynchronize(c->stream));
+  if (bad[0]) return fail(2, "%d appended factor(s) reference a stamp outside the spline's valid range or an invalid camera / landmark", bad[0]);
+  if (bad[1]) return fail(3, "appended factors must arrive in stamp order (%d fall before the end of the list): use hb200_set_*_factors + hb200_bind", bad[1]);
+  return 0;
+}
+
+// grow the visual list to Nv + n entries, the first Nv preserved (the buffers may move: the captured iteration goes)
+int grow_visual(hb200_ctx* c, size_t Nv, size_t n) {
+  c->graph_valid = false;
+  HB_CUDA(c->v_stamp.grow(Nv + n, Nv, c->stream)); HB_CUDA(c->v_pixel.grow(2 * (Nv + n), 2 * Nv, c->stream));
+  HB_CUDA(c->v_z.grow(Nv + n, Nv, c->stream)); HB_CUDA(c->v_idx.grow(Nv + n, Nv, c->stream));
   return 0;
 }
 }  // namespace
@@ -2297,7 +2350,7 @@ int hb200_append_pixel_factors(hb200_ctx* c, int n, const double* stamp, const i
   if (n <= 0 || !stamp || !camera || !landmark || !pixel) return fail(-1, "invalid pixel factors");
   HB_CUDA(cudaSetDevice(c->device));
   const size_t Nv = c->Nv;
-  HB_CUDA(c->v_stamp.grow(Nv + n, Nv, c->stream)); HB_CUDA(c->v_pixel.grow(2 * (Nv + n), 2 * Nv, c->stream)); HB_CUDA(c->v_idx.grow(Nv + n, Nv, c->stream));
+  if ((rc = grow_visual(c, Nv, n))) return rc;
   DevBuf<int> d_cam, d_lm;
   HB_CUDA(d_cam.ensure(n)); HB_CUDA(d_lm.ensure(n));
   HB_CUDA(c->d_invalid.ensure(2));
@@ -2306,16 +2359,119 @@ int hb200_append_pixel_factors(hb200_ctx* c, int n, const double* stamp, const i
   HB_CUDA(cudaMemcpyAsync(c->v_pixel.p + 2 * Nv, pixel, sizeof(double) * 2 * n, cudaMemcpyHostToDevice, c->stream));
   HB_CUDA(cudaMemcpyAsync(d_cam.p, camera, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
   HB_CUDA(cudaMemcpyAsync(d_lm.p, landmark, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
-  bind_pixel_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, c->v_stamp.p + Nv, d_cam.p, d_lm.p, c->knots[0].p, c->K, c->k, c->C, c->L, c->v_idx.p + Nv, c->d_invalid.p);
+  bind_pixel_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, c->v_stamp.p + Nv, d_cam.p, d_lm.p, c->knots[0].p, c->K, c->k, c->C, c->L, 0, c->v_idx.p + Nv, c->d_invalid.p);
   HB_LAUNCH(c, "bind_pixel_kernel");
-  tail_sorted_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(static_cast<int>(Nv), n, c->v_idx.p, c->d_invalid.p + 1);
+  if ((rc = check_visual_tail(c, static_cast<int>(Nv), n))) return rc;
+  c->Nv = static_cast<int>(Nv) + n; c->Np += n;
+  return rebuild_incidence_device(c);
+}
+
+int hb200_append_bearing_factors(hb200_ctx* c, int n, const double* stamp, const int* camera, const int* landmark, const double* bearing) {
+  int rc = check_device_window(c);
+  if (rc) return rc;
+  if (n <= 0 || !stamp || !camera || !landmark || !bearing) return fail(-1, "invalid bearing factors");
+  HB_CUDA(cudaSetDevice(c->device));
+  const size_t Nv = c->Nv;
+  if ((rc = grow_visual(c, Nv, n))) return rc;
+  // [n][3] -> the visual list's (x, y) pairs + z column
+  std::vector<double> xy(2 * static_cast<size_t>(n)), z(n);
+  for (int f = 0; f < n; ++f) { xy[2 * f] = bearing[3 * f]; xy[2 * f + 1] = bearing[3 * f + 1]; z[f] = bearing[3 * f + 2]; }
+  DevBuf<int> d_cam, d_lm;
+  HB_CUDA(d_cam.ensure(n)); HB_CUDA(d_lm.ensure(n));
+  HB_CUDA(c->d_invalid.ensure(2));
+  HB_CUDA(cudaMemsetAsync(c->d_invalid.p, 0, 2 * sizeof(int), c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->v_stamp.p + Nv, stamp, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->v_pixel.p + 2 * Nv, xy.data(), sizeof(double) * 2 * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->v_z.p + Nv, z.data(), sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(d_cam.p, camera, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(d_lm.p, landmark, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+  bind_pixel_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, c->v_stamp.p + Nv, d_cam.p, d_lm.p, c->knots[0].p, c->K, c->k, c->C, c->L, 1, c->v_idx.p + Nv, c->d_invalid.p);
+  HB_LAUNCH(c, "bind_pixel_kernel");
+  if ((rc = check_visual_tail(c, static_cast<int>(Nv), n))) return rc;
+  c->Nv = static_cast<int>(Nv) + n; c->Nb += n;
+  return rebuild_incidence_device(c);
+}
+
+int hb200_append_manifold_factors(hb200_ctx* c, int n, const double* stamp, const int* sensor, const double* pose) {
+  int rc = check_device_window(c);
+  if (rc) return rc;
+  if (n <= 0 || !stamp || !sensor || !pose) return fail(-1, "invalid manifold factors");
+  if (c->P == 0) return fail(-2, "manifold factors need pose sensors (hb200_set_pose_sensors)");
+  HB_CUDA(cudaSetDevice(c->device));
+  const size_t Nm = c->Nm;
+  c->graph_valid = false;   // (the buffers may move)
+  HB_CUDA(c->m_stamp.grow(Nm + n, Nm, c->stream)); HB_CUDA(c->m_meas.grow(7 * (Nm + n), 7 * Nm, c->stream)); HB_CUDA(c->m_idx.grow(Nm + n, Nm, c->stream));
+  HB_CUDA(c->m_sensor.ensure(n));
+  HB_CUDA(c->d_invalid.ensure(2));
+  HB_CUDA(cudaMemsetAsync(c->d_invalid.p, 0, 2 * sizeof(int), c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->m_stamp.p + Nm, stamp, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->m_meas.p + 7 * Nm, pose, sizeof(double) * 7 * n, cudaMemcpyHostToDevice, c->stream));
+  HB_CUDA(cudaMemcpyAsync(c->m_sensor.p, sensor, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+  bind_manifold_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, c->m_stamp.p + Nm, c->m_sensor.p, c->knots[0].p, c->K, c->k, c->P, c->m_idx.p + Nm, c->d_invalid.p);
+  HB_LAUNCH(c, "bind_manifold_kernel");
+  tail_sorted_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(static_cast<int>(Nm), n, c->m_idx.p, c->d_invalid.p + 1);
   HB_LAUNCH(c, "tail_sorted_kernel");
   int bad[2] = {0, 0};
   HB_CUDA(cudaMemcpyAsync(bad, c->d_invalid.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   HB_CUDA(cudaStreamSynchronize(c->stream));
-  if (bad[0]) return fail(2, "%d appended factor(s) reference a stamp outside the spline's valid range or an invalid camera / landmark", bad[0]);
-  if (bad[1]) return fail(3, "appended factors must arrive in stamp order (%d fall before the end of the list): use hb200_set_pixel_factors + hb200_bind", bad[1]);
-  c->Nv = static_cast<int>(Nv) + n; c->Np = c->Nv;
+  if (bad[0]) return fail(2, "%d appended pose factor(s) reference a stamp outside the spline's valid range or an invalid sensor", bad[0]);
+  if (bad[1]) return fail(3, "appended factors must arrive in stamp order (%d fall before the end of the list): use hb200_set_manifold_factors + hb200_bind", bad[1]);
+  c->Nm = static_cast<int>(Nm) + n;
+  return rebuild_incidence_device(c);
+}
+
+int hb200_append_stereo_tracks(hb200_ctx* c, int n, const double* stamp, const int* camera0, const int* camera1, const double* pixel0,
+                               const double* pixel1, const int* landmark_in, int* landmark_out, int* num_new) {
+  int rc = check_device_window(c);
+  if (rc) return rc;
+  if (n <= 0 || !stamp || !camera0 || !camera1 || !pixel0 || !pixel1 || !landmark_in) return fail(-1, "invalid stereo tracks");
+  if (c->C == 0) return fail(-2, "cameras not set");
+  if (c->k != 4 && c->k != 6) return fail(-4, "spline order %d not supported (4 or 6)", c->k);
+  HB_CUDA(cudaSetDevice(c->device));
+  const size_t N = n, Nv = c->Nv, L = c->L;
+  // one H2D copy: [pixel0 2n | pixel1 2n | stamp n] doubles (the pixel pairs 16-byte aligned), then
+  // [camera0 n | camera1 n | landmark_in n] ints
+  const size_t nd = 5 * N, ni = 3 * N;
+  std::vector<double> stage(nd + (ni + 1) / 2);
+  std::memcpy(stage.data(), pixel0, sizeof(double) * 2 * N);
+  std::memcpy(stage.data() + 2 * N, pixel1, sizeof(double) * 2 * N);
+  std::memcpy(stage.data() + 4 * N, stamp, sizeof(double) * N);
+  int* si = reinterpret_cast<int*>(stage.data() + nd);
+  std::memcpy(si, camera0, sizeof(int) * N); std::memcpy(si + N, camera1, sizeof(int) * N); std::memcpy(si + 2 * N, landmark_in, sizeof(int) * N);
+  DevBuf<double> d_in;
+  DevBuf<int> d_flag, d_pos, d_out;   // d_out: [invalid, out of order, new landmarks | landmark_out n]
+  HB_CUDA(d_in.ensure(stage.size())); HB_CUDA(d_flag.ensure(N)); HB_CUDA(d_pos.ensure(N)); HB_CUDA(d_out.ensure(3 + N));
+  if ((rc = grow_visual(c, Nv, 2 * N))) return rc;
+  for (int s2 = 0; s2 < 2; ++s2) HB_CUDA(c->lms[s2].grow(3 * (L + N), s2 == 0 ? 3 * L : 0, c->stream));
+  HB_CUDA(cudaMemsetAsync(d_out.p, 0, 3 * sizeof(int), c->stream));
+  HB_CUDA(cudaMemcpyAsync(d_in.p, stage.data(), sizeof(double) * stage.size(), cudaMemcpyHostToDevice, c->stream));
+  const int* d_i = reinterpret_cast<const int*>(d_in.p + nd);
+  stereo_new_flags_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(n, d_i + 2 * N, c->L, d_flag.p, d_out.p);
+  HB_LAUNCH(c, "stereo_new_flags_kernel");
+  scan_kernel<<<1, 1024, 0, c->stream>>>(d_flag.p, n, d_pos.p, d_out.p + 2);
+  HB_LAUNCH(c, "scan_kernel");
+  prep_kernel<<<(c->K + 63) / 64, 64, 0, c->stream>>>(c->K, c->knots[0].p, c->tab[0].p, nullptr, 0);
+  HB_LAUNCH(c, "prep_kernel");
+  const double2* q0 = reinterpret_cast<const double2*>(d_in.p);
+  const double2* q1 = reinterpret_cast<const double2*>(d_in.p + 2 * N);
+  double2* vpx = reinterpret_cast<double2*>(c->v_pixel.p);
+  if (c->k == 4)
+    append_stereo_tracks_kernel<4><<<(n + 127) / 128, 128, 0, c->stream>>>(n, d_in.p + 4 * N, q0, q1, d_i, d_i + N, d_i + 2 * N, d_pos.p, c->knots[0].p, c->tab[0].p, c->K, c->basis,
+                                                                       c->cams.p, c->C, c->L, c->Nv, c->v_stamp.p, vpx, c->v_z.p, c->v_idx.p, c->lms[0].p, d_out.p + 3, d_out.p);
+  else
+    append_stereo_tracks_kernel<6><<<(n + 127) / 128, 128, 0, c->stream>>>(n, d_in.p + 4 * N, q0, q1, d_i, d_i + N, d_i + 2 * N, d_pos.p, c->knots[0].p, c->tab[0].p, c->K, c->basis,
+                                                                       c->cams.p, c->C, c->L, c->Nv, c->v_stamp.p, vpx, c->v_z.p, c->v_idx.p, c->lms[0].p, d_out.p + 3, d_out.p);
+  HB_LAUNCH(c, "append_stereo_tracks_kernel");
+  tail_sorted_kernel<<<(2 * n + 127) / 128, 128, 0, c->stream>>>(static_cast<int>(Nv), 2 * n, c->v_idx.p, d_out.p + 1);
+  HB_LAUNCH(c, "tail_sorted_kernel");
+  std::vector<int> h(3 + N);
+  HB_CUDA(cudaMemcpyAsync(h.data(), d_out.p, sizeof(int) * (3 + N), cudaMemcpyDeviceToHost, c->stream));
+  HB_CUDA(cudaStreamSynchronize(c->stream));
+  if (h[0]) return fail(2, "%d stereo track(s) reference a stamp outside the spline's valid range, an invalid camera or a landmark slot outside [-1, L)", h[0]);
+  if (h[1]) return fail(3, "appended factors must arrive in stamp order (%d fall before the end of the list): use hb200_set_bearing_factors + hb200_bind", h[1]);
+  if (landmark_out) std::memcpy(landmark_out, h.data() + 3, sizeof(int) * N);
+  if (num_new) *num_new = h[2];
+  c->Nv = static_cast<int>(Nv + 2 * N); c->Nb += 2 * n; c->L = static_cast<int>(L) + h[2];
   return rebuild_incidence_device(c);
 }
 
@@ -2349,19 +2505,21 @@ int hb200_slide(hb200_ctx* c, double lower_bound, int flags, hb200_slide_stats* 
   int rc = check_device_window(c);
   if (rc) return rc;
   HB_CUDA(cudaSetDevice(c->device));
-  const int Nv = c->Nv, Ni = c->Ni, L = c->L, K = c->K;
+  const int Nv = c->Nv, Ni = c->Ni, Nm = c->Nm, L = c->L, K = c->K;
   // knot index of the last state element at or before the lower bound; the window keeps `left padding` elements in
   // front of the one that starts the lower bound's interval (reference optimizer.cpp:289: prev(upper_bound(lower), left_padding))
   int ub = static_cast<int>(std::upper_bound(c->h_knot_stamp.begin(), c->h_knot_stamp.end(), lower_bound) - c->h_knot_stamp.begin());
   const int begin = std::max(0, ub - 1 - (c->k - 1) / 2);
   const int last_const = ub - 1;   // knots 0 .. last_const have stamp <= lower bound
   HB_CUDA(c->w_scal.ensure(8));
-  int init[8] = {0, 0, 0, 0x7fffffff, 0x7fffffff, 0, 0, 0};   // [L_new, Nv_new, Ni_new, min base visual, min base inertial]
+  // [L_new, Nv_new, Ni_new, min base visual, min base inertial, min base manifold, bearing factors kept, Nm_new]
+  int init[8] = {0, 0, 0, 0x7fffffff, 0x7fffffff, 0x7fffffff, 0, 0};
   HB_CUDA(cudaMemcpyAsync(c->w_scal.p, init, sizeof(init), cudaMemcpyHostToDevice, c->stream));
   HB_CUDA(c->w_last.ensure(std::max(L, 1))); HB_CUDA(c->w_lkeep.ensure(std::max(L, 1) + 1)); HB_CUDA(c->w_lpos.ensure(std::max(L, 1) + 1));
   HB_CUDA(c->w_keep.ensure(std::max(std::max(Nv, Ni), 1))); HB_CUDA(c->w_pos.ensure(std::max(std::max(Nv, Ni), 1)));
-  DevBuf<int> i_keep, i_pos;
+  DevBuf<int> i_keep, i_pos, m_keep, m_pos;
   HB_CUDA(i_keep.ensure(std::max(Ni, 1))); HB_CUDA(i_pos.ensure(std::max(Ni, 1)));
+  if (Nm) { HB_CUDA(m_keep.ensure(Nm)); HB_CUDA(m_pos.ensure(Nm)); }
   HB_CUDA(cudaMemsetAsync(c->w_last.p, 0, sizeof(unsigned long long) * std::max(L, 1), c->stream));
   if (Nv) { landmark_last_stamp_kernel<<<(Nv + 255) / 256, 256, 0, c->stream>>>(Nv, c->v_stamp.p, c->v_idx.p, c->w_last.p); HB_LAUNCH(c, "landmark_last_stamp_kernel"); }
   if (L) {
@@ -2371,7 +2529,7 @@ int hb200_slide(hb200_ctx* c, double lower_bound, int flags, hb200_slide_stats* 
     HB_LAUNCH(c, "scan_kernel");
   }
   if (Nv) {
-    visual_keep_kernel<<<(Nv + 255) / 256, 256, 0, c->stream>>>(Nv, c->v_idx.p, c->w_lkeep.p, c->w_keep.p, c->w_scal.p + 3);
+    visual_keep_kernel<<<(Nv + 255) / 256, 256, 0, c->stream>>>(Nv, c->v_idx.p, c->w_lkeep.p, c->w_keep.p, c->w_scal.p + 3, c->w_scal.p + 6);
     HB_LAUNCH(c, "visual_keep_kernel");
     scan_kernel<<<1, 1024, 0, c->stream>>>(c->w_keep.p, Nv, c->w_pos.p, c->w_scal.p + 1);
     HB_LAUNCH(c, "scan_kernel");
@@ -2382,33 +2540,48 @@ int hb200_slide(hb200_ctx* c, double lower_bound, int flags, hb200_slide_stats* 
     scan_kernel<<<1, 1024, 0, c->stream>>>(i_keep.p, Ni, i_pos.p, c->w_scal.p + 2);
     HB_LAUNCH(c, "scan_kernel");
   }
+  if (Nm) {
+    manifold_keep_kernel<<<(Nm + 255) / 256, 256, 0, c->stream>>>(Nm, c->m_idx.p, c->k, (flags & HB200_SLIDE_DROP_POSE) ? last_const : -1, m_keep.p, c->w_scal.p + 5);
+    HB_LAUNCH(c, "manifold_keep_kernel");
+    scan_kernel<<<1, 1024, 0, c->stream>>>(m_keep.p, Nm, m_pos.p, c->w_scal.p + 7);
+    HB_LAUNCH(c, "scan_kernel");
+  }
   int h[8];
   HB_CUDA(cudaMemcpyAsync(h, c->w_scal.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
   HB_CUDA(cudaStreamSynchronize(c->stream));
-  const int L_new = L ? h[0] : 0, Nv_new = Nv ? h[1] : 0, Ni_new = Ni ? h[2] : 0;
+  const int L_new = L ? h[0] : 0, Nv_new = Nv ? h[1] : 0, Ni_new = Ni ? h[2] : 0, Nm_new = Nm ? h[7] : 0, Nb_new = h[6];
   // state elements in front of `begin` go once no residual touches them (reference optimizer.cpp:331-341)
-  int shift = std::min(begin, std::min(h[3], h[4]));
+  int shift = std::min(std::min(begin, h[5]), std::min(h[3], h[4]));
   shift = std::max(0, std::min(shift, K - c->k));
   const int K_new = K - shift;
   // compaction into the alternate buffers, then swap
-  HB_CUDA(c->alt_stamp.ensure(std::max(std::max(Nv_new, Ni_new), 1))); HB_CUDA(c->alt_idx.ensure(std::max(std::max(Nv_new, Ni_new), 1)));
-  HB_CUDA(c->alt_pixel.ensure(std::max(Nv_new, 1)));
+  HB_CUDA(c->alt_stamp.ensure(std::max(std::max(Nv_new, Ni_new), std::max(Nm_new, 1)))); HB_CUDA(c->alt_idx.ensure(std::max(std::max(Nv_new, Ni_new), 1)));
+  HB_CUDA(c->alt_meas.ensure(std::max(6 * static_cast<size_t>(Ni_new), 7 * static_cast<size_t>(std::max(Nm_new, 1)))));
+  HB_CUDA(c->alt_midx.ensure(std::max(Nm_new, 1)));
+  HB_CUDA(c->alt_pixel.ensure(std::max(Nv_new, 1))); HB_CUDA(c->alt_z.ensure(std::max(Nv_new, 1)));
   if (Nv) {
     compact_visual_kernel<<<(Nv + 255) / 256, 256, 0, c->stream>>>(Nv, c->w_keep.p, c->w_pos.p, c->w_lpos.p, shift, c->v_stamp.p, reinterpret_cast<const double2*>(c->v_pixel.p),
-                                                                  c->v_idx.p, c->alt_stamp.p, c->alt_pixel.p, c->alt_idx.p);
+                                                                  c->v_z.p, c->v_idx.p, c->alt_stamp.p, c->alt_pixel.p, c->alt_z.p, c->alt_idx.p);
     HB_LAUNCH(c, "compact_visual_kernel");
     // (v_pixel is a DevBuf<double>: copy the compacted pairs back instead of swapping differently typed buffers)
     HB_CUDA(cudaMemcpyAsync(c->v_pixel.p, c->alt_pixel.p, sizeof(double2) * Nv_new, cudaMemcpyDeviceToDevice, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->v_stamp.p, c->alt_stamp.p, sizeof(double) * Nv_new, cudaMemcpyDeviceToDevice, c->stream));
+    if (c->Nb) HB_CUDA(cudaMemcpyAsync(c->v_z.p, c->alt_z.p, sizeof(double) * Nv_new, cudaMemcpyDeviceToDevice, c->stream));   // (read for bearings only)
     HB_CUDA(cudaMemcpyAsync(c->v_idx.p, c->alt_idx.p, sizeof(int4) * Nv_new, cudaMemcpyDeviceToDevice, c->stream));
   }
   if (Ni) {
-    HB_CUDA(c->alt_meas.ensure(6 * static_cast<size_t>(std::max(Ni_new, 1))));
     compact_inertial_kernel<<<(Ni + 255) / 256, 256, 0, c->stream>>>(Ni, i_keep.p, i_pos.p, shift, c->i_stamp.p, c->i_meas.p, c->i_idx.p, c->alt_stamp.p, c->alt_meas.p, c->alt_idx.p);
     HB_LAUNCH(c, "compact_inertial_kernel");
     HB_CUDA(cudaMemcpyAsync(c->i_stamp.p, c->alt_stamp.p, sizeof(double) * Ni_new, cudaMemcpyDeviceToDevice, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->i_meas.p, c->alt_meas.p, sizeof(double) * 6 * Ni_new, cudaMemcpyDeviceToDevice, c->stream));
     HB_CUDA(cudaMemcpyAsync(c->i_idx.p, c->alt_idx.p, sizeof(int4) * Ni_new, cudaMemcpyDeviceToDevice, c->stream));
+  }
+  if (Nm) {
+    compact_manifold_kernel<<<(Nm + 255) / 256, 256, 0, c->stream>>>(Nm, m_keep.p, m_pos.p, shift, c->m_stamp.p, c->m_meas.p, c->m_idx.p, c->alt_stamp.p, c->alt_meas.p, c->alt_midx.p);
+    HB_LAUNCH(c, "compact_manifold_kernel");
+    HB_CUDA(cudaMemcpyAsync(c->m_stamp.p, c->alt_stamp.p, sizeof(double) * Nm_new, cudaMemcpyDeviceToDevice, c->stream));
+    HB_CUDA(cudaMemcpyAsync(c->m_meas.p, c->alt_meas.p, sizeof(double) * 7 * Nm_new, cudaMemcpyDeviceToDevice, c->stream));
+    HB_CUDA(cudaMemcpyAsync(c->m_idx.p, c->alt_midx.p, sizeof(int2) * Nm_new, cudaMemcpyDeviceToDevice, c->stream));
   }
   if (L) {
     HB_CUDA(c->alt_lms.ensure(3 * static_cast<size_t>(std::max(L_new, 1))));
@@ -2429,13 +2602,22 @@ int hb200_slide(hb200_ctx* c, double lower_bound, int flags, hb200_slide_stats* 
   c->h_knot_const.assign(K_new, 0);
   for (int j = 0; j < K_new; ++j) c->h_knot_const[j] = c->h_knot_stamp[j] <= lower_bound ? 1 : 0;
   if (ub > 0) c->gravity_const = 1;
-  c->K = K_new; c->L = L_new; c->Nv = Nv_new; c->Np = Nv_new; c->Ni = Ni_new;
+  c->K = K_new; c->L = L_new; c->Nv = Nv_new; c->Np = Nv_new - Nb_new; c->Nb = Nb_new; c->Ni = Ni_new; c->Nm = Nm_new;
   if (stats) {
     stats->knots_dropped = shift; stats->knots_constant = std::max(0, ub - shift); stats->landmarks_dropped = L - L_new;
     stats->visual_factors_dropped = Nv - Nv_new; stats->inertial_factors_dropped = Ni - Ni_new;
     stats->knots = K_new; stats->landmarks = L_new; stats->visual_factors = Nv_new; stats->inertial_factors = Ni_new;
   }
   return rebuild_incidence_device(c);
+}
+
+int hb200_factor_counts(hb200_ctx* c, int* pixel, int* bearing, int* inertial, int* manifold) {
+  if (!c) return fail(-1, "null context");
+  if (pixel) *pixel = c->Np;
+  if (bearing) *bearing = c->Nb;
+  if (inertial) *inertial = c->Ni;
+  if (manifold) *manifold = c->Nm;
+  return 0;
 }
 
 int hb200_window_sizes(hb200_ctx* c, int* knots, int* landmarks, int* visual_factors, int* inertial_factors) {

@@ -90,14 +90,15 @@ HB_DI int segment_base(const double* knots, int stride, int stamp_off, int K, in
   return base;
 }
 
+// pixel and bearing factors share the visual list: `kind` (0 pixel, 1 bearing) goes to idx.w
 __global__ void bind_pixel_kernel(int n, const double* __restrict__ stamp, const int* __restrict__ cam, const int* __restrict__ lm,
-                                  const double* __restrict__ knots, int K, int k, int C, int L, int4* __restrict__ idx,
+                                  const double* __restrict__ knots, int K, int k, int C, int L, int kind, int4* __restrict__ idx,
                                   int* __restrict__ num_invalid) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= n) return;
   const int base = segment_base(knots, 8, 7, K, k, stamp[f]);
   const int c = cam[f], l = lm[f];
-  idx[f] = make_int4(base, l, c, 0);
+  idx[f] = make_int4(base, l, c, kind);
   if (base < 0 || c < 0 || c >= C || l < 0 || l >= L) atomicAdd(num_invalid, 1);
 }
 
@@ -1216,22 +1217,15 @@ HB_DI void pixel_to_bearing(const double* __restrict__ cam /* raw [T_bs 7 | cx c
   b[0] = x * inv; b[1] = y * inv; b[2] = inv;
 }
 
+// One stereo track: bearings b0 / b1 of both views and the triangulated world landmark lm at the state's pose at t.
+// Returns the knot base of t, or -1 (outputs untouched) when the stamp or a camera index is invalid.  Shared by
+// ingest_stereo_kernel and append_stereo_tracks_kernel (hb200_window.cuh); not inlined, so that both kernels run the
+// same compiled code and produce the same bits (inlined, the two copies may contract multiply-adds differently).
 template <int K>
-__global__ void ingest_stereo_kernel(int n, const double* __restrict__ stamps, const int* __restrict__ cam0, const int* __restrict__ cam1,
-                                     const double* __restrict__ px0, const double* __restrict__ px1, const double* __restrict__ knots,
-                                     const double* __restrict__ tab, int Kn, Basis B, const double* __restrict__ cams, int C,
-                                     double* __restrict__ b0_out, double* __restrict__ b1_out, double* __restrict__ lm_out,
-                                     int* __restrict__ num_invalid) {
-  const int f = blockIdx.x * blockDim.x + threadIdx.x;
-  if (f >= n) return;
-  const double t = stamps[f];
+__device__ __noinline__ int ingest_stereo_track(double t, int c0, int c1, double2 q0, double2 q1, const double* __restrict__ knots, const double* __restrict__ tab,
+                              int Kn, const Basis& B, const double* __restrict__ cams, int C, double* b0, double* b1, double* lm) {
   const int base = segment_base(knots, 8, 7, Kn, K, t);
-  const int c0 = cam0[f], c1 = cam1[f];
-  if (base < 0 || c0 < 0 || c0 >= C || c1 < 0 || c1 >= C) {
-    atomicAdd(num_invalid, 1);
-    for (int i = 0; i < 3; ++i) { b0_out[3 * static_cast<size_t>(f) + i] = 0.0; b1_out[3 * static_cast<size_t>(f) + i] = 0.0; lm_out[3 * static_cast<size_t>(f) + i] = 0.0; }
-    return;
-  }
+  if (base < 0 || c0 < 0 || c0 >= C || c1 < 0 || c1 >= C) return -1;
   // pose of the body at the stamp (value only)
   constexpr int left = (K - 1) / 2;
   const double* row0 = tab + static_cast<size_t>(base) * kTabStride;
@@ -1257,9 +1251,8 @@ __global__ void ingest_stereo_kernel(int n, const double* __restrict__ stamps, c
   }
   const double* ca = cams + 15 * static_cast<size_t>(c0);
   const double* cb = cams + 15 * static_cast<size_t>(c1);
-  double b0[3], b1[3];
-  pixel_to_bearing(ca, px0[2 * static_cast<size_t>(f)], px0[2 * static_cast<size_t>(f) + 1], b0);
-  pixel_to_bearing(cb, px1[2 * static_cast<size_t>(f)], px1[2 * static_cast<size_t>(f) + 1], b1);
+  pixel_to_bearing(ca, q0.x, q0.y, b0);
+  pixel_to_bearing(cb, q1.x, q1.y, b1);
   // T_01 = T_b0^-1 (+) T_b1: R_01 = R_b0^T R_b1, t_01 = R_b0^T (t_b1 - t_b0)
   double Ra[9], Rb[9], R01[9], d1[3], t01[3];
   quat_to_rot(ca, Ra);
@@ -1281,10 +1274,27 @@ __global__ void ingest_stereo_kernel(int n, const double* __restrict__ stamps, c
   pb[0] += ca[4]; pb[1] += ca[5]; pb[2] += ca[6];
   m3_vec(R, pb, pw);
 #pragma unroll
+  for (int i = 0; i < 3; ++i) lm[i] = pw[i] + p[i];
+  return base;
+}
+
+template <int K>
+__global__ void ingest_stereo_kernel(int n, const double* __restrict__ stamps, const int* __restrict__ cam0, const int* __restrict__ cam1,
+                                     const double* __restrict__ px0, const double* __restrict__ px1, const double* __restrict__ knots,
+                                     const double* __restrict__ tab, int Kn, Basis B, const double* __restrict__ cams, int C,
+                                     double* __restrict__ b0_out, double* __restrict__ b1_out, double* __restrict__ lm_out,
+                                     int* __restrict__ num_invalid) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  const double2 q0 = make_double2(px0[2 * static_cast<size_t>(f)], px0[2 * static_cast<size_t>(f) + 1]);
+  const double2 q1 = make_double2(px1[2 * static_cast<size_t>(f)], px1[2 * static_cast<size_t>(f) + 1]);
+  double b0[3] = {0.0, 0.0, 0.0}, b1[3] = {0.0, 0.0, 0.0}, lm[3] = {0.0, 0.0, 0.0};
+  if (ingest_stereo_track<K>(stamps[f], cam0[f], cam1[f], q0, q1, knots, tab, Kn, B, cams, C, b0, b1, lm) < 0) atomicAdd(num_invalid, 1);
+#pragma unroll
   for (int i = 0; i < 3; ++i) {
     b0_out[3 * static_cast<size_t>(f) + i] = b0[i];
     b1_out[3 * static_cast<size_t>(f) + i] = b1[i];
-    lm_out[3 * static_cast<size_t>(f) + i] = pw[i] + p[i];
+    lm_out[3 * static_cast<size_t>(f) + i] = lm[i];
   }
 }
 

@@ -65,13 +65,17 @@ __global__ void landmark_keep_kernel(int L, const unsigned long long* __restrict
   const int l = blockIdx.x * blockDim.x + threadIdx.x;
   if (l < L) keep[l] = (last[l] == 0ull || stamp_from_key(last[l]) >= lower) ? 1 : 0;
 }
-// visual factors live and die with their landmark; min_base receives the smallest knot base among the kept ones
-__global__ void visual_keep_kernel(int n, const int4* __restrict__ idx, const int* __restrict__ lm_keep, int* __restrict__ keep, int* __restrict__ min_base) {
+// visual factors live and die with their landmark; min_base receives the smallest knot base among the kept ones,
+// bearing_kept the number of kept bearing factors (kind 1)
+__global__ void visual_keep_kernel(int n, const int4* __restrict__ idx, const int* __restrict__ lm_keep, int* __restrict__ keep, int* __restrict__ min_base,
+                                   int* __restrict__ bearing_kept) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= n) return;
-  const int k = lm_keep[idx[f].y];
+  const int4 id = idx[f];
+  const int k = lm_keep[id.y];
   keep[f] = k;
-  if (k) atomicMin(min_base, idx[f].x);
+  if (k) atomicMin(min_base, id.x);
+  if (k && id.w) atomicAdd(bearing_kept, 1);
 }
 // inertial factors: kept (the reference never removes them); with drop_base >= 0 those whose control points ALL lie
 // at or before the lower bound (base + order - 1 <= drop_base: every block the residual moves with is constant) go
@@ -83,15 +87,38 @@ __global__ void inertial_keep_kernel(int n, const int4* __restrict__ idx, int or
   if (k) atomicMin(min_base, idx[f].x);
 }
 
+// pose priors (manifold factors): kept, as in the reference; with drop_base >= 0 the same rule as inertial_keep_kernel
+__global__ void manifold_keep_kernel(int n, const int2* __restrict__ idx, int order, int drop_base, int* __restrict__ keep, int* __restrict__ min_base) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  const int k = (drop_base >= 0 && idx[f].x + order - 1 <= drop_base) ? 0 : 1;
+  keep[f] = k;
+  if (k) atomicMin(min_base, idx[f].x);
+}
+
+// (z: third component of a bearing measurement; pixel factors carry 0 there)
 __global__ void compact_visual_kernel(int n, const int* __restrict__ keep, const int* __restrict__ pos, const int* __restrict__ lm_pos, int knot_shift,
-                                      const double* __restrict__ stamp, const double2* __restrict__ pixel, const int4* __restrict__ idx,
-                                      double* __restrict__ stamp_o, double2* __restrict__ pixel_o, int4* __restrict__ idx_o) {
+                                      const double* __restrict__ stamp, const double2* __restrict__ pixel, const double* __restrict__ z,
+                                      const int4* __restrict__ idx, double* __restrict__ stamp_o, double2* __restrict__ pixel_o,
+                                      double* __restrict__ z_o, int4* __restrict__ idx_o) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= n || !keep[f]) return;
   const int p = pos[f];
   int4 id = idx[f];
   id.x -= knot_shift; id.y = lm_pos[id.y];
-  stamp_o[p] = stamp[f]; pixel_o[p] = pixel[f]; idx_o[p] = id;
+  stamp_o[p] = stamp[f]; pixel_o[p] = pixel[f]; z_o[p] = z[f]; idx_o[p] = id;
+}
+__global__ void compact_manifold_kernel(int n, const int* __restrict__ keep, const int* __restrict__ pos, int knot_shift, const double* __restrict__ stamp,
+                                        const double* __restrict__ meas, const int2* __restrict__ idx, double* __restrict__ stamp_o,
+                                        double* __restrict__ meas_o, int2* __restrict__ idx_o) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n || !keep[f]) return;
+  const int p = pos[f];
+  int2 id = idx[f];
+  id.x -= knot_shift;
+  stamp_o[p] = stamp[f]; idx_o[p] = id;
+#pragma unroll
+  for (int q = 0; q < 7; ++q) meas_o[7 * static_cast<size_t>(p) + q] = meas[7 * static_cast<size_t>(f) + q];
 }
 __global__ void compact_inertial_kernel(int n, const int* __restrict__ keep, const int* __restrict__ pos, int knot_shift, const double* __restrict__ stamp,
                                         const double* __restrict__ meas, const int4* __restrict__ idx, double* __restrict__ stamp_o,
@@ -168,9 +195,49 @@ __global__ void run_fill_kernel(int n, const int* __restrict__ flag, const int* 
   if (f == 0) run_off[nruns] = n;
 }
 // bound-order check of an appended tail: every new base must be >= the last old one and the tail itself ascending
-__global__ void tail_sorted_kernel(int n_old, int n_new, const int4* __restrict__ idx, int* __restrict__ bad) {
+// (Idx = int4 for the visual / inertial lists, int2 for the manifold list: the base is .x in all of them)
+template <typename Idx>
+__global__ void tail_sorted_kernel(int n_old, int n_new, const Idx* __restrict__ idx, int* __restrict__ bad) {
   const int f = n_old + blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= n_old + n_new || f == 0) return;
   if (idx[f].x < idx[f - 1].x) atomicAdd(bad, 1);
+}
+
+// ---- stereo tracks (reference abstract.cpp:243-260: process(VisualTracks)) ----------------------------------------
+// "new landmark" flags of the tracks (landmark_in == -1); any other value must be an existing window slot
+__global__ void stereo_new_flags_kernel(int n, const int* __restrict__ lm_in, int L, int* __restrict__ flag, int* __restrict__ num_invalid) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int l = lm_in[i];
+  flag[i] = (l == -1) ? 1 : 0;
+  if (l < -1 || l >= L) atomicAdd(num_invalid, 1);
+}
+// One thread per track: bearings of both views and, for a new landmark, the triangulated point at the current state
+// (ingest_stereo_track).  Writes the two bearing factors of track i -- camera0's at Nv + 2i, camera1's at Nv + 2i + 1 --
+// straight into the grown visual list (kind 1), and a new landmark into slot L + new_pos[i] of `lms`.  lm_out[i]
+// receives the slot the track's factors reference.  Invalid tracks are counted; the caller then discards the tail.
+template <int K>
+__global__ void append_stereo_tracks_kernel(int n, const double* __restrict__ stamp, const double2* __restrict__ px0, const double2* __restrict__ px1,
+                                            const int* __restrict__ cam0, const int* __restrict__ cam1, const int* __restrict__ lm_in,
+                                            const int* __restrict__ new_pos, const double* __restrict__ knots, const double* __restrict__ tab, int Kn, Basis B,
+                                            const double* __restrict__ cams, int C, int L, int Nv, double* __restrict__ v_stamp, double2* __restrict__ v_pixel,
+                                            double* __restrict__ v_z, int4* __restrict__ v_idx, double* __restrict__ lms, int* __restrict__ lm_out,
+                                            int* __restrict__ num_invalid) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double t = stamp[i];
+  const int c0 = cam0[i], c1 = cam1[i], li = lm_in[i];
+  const int l = (li == -1) ? L + new_pos[i] : li;
+  double b0[3] = {0.0, 0.0, 0.0}, b1[3] = {0.0, 0.0, 0.0}, p[3] = {0.0, 0.0, 0.0};
+  const int base = ingest_stereo_track<K>(t, c0, c1, px0[i], px1[i], knots, tab, Kn, B, cams, C, b0, b1, p);
+  if (base < 0) atomicAdd(num_invalid, 1);
+  const size_t f = static_cast<size_t>(Nv) + 2 * static_cast<size_t>(i);
+  v_stamp[f] = t; v_pixel[f] = make_double2(b0[0], b0[1]); v_z[f] = b0[2]; v_idx[f] = make_int4(base, l, c0, 1);
+  v_stamp[f + 1] = t; v_pixel[f + 1] = make_double2(b1[0], b1[1]); v_z[f + 1] = b1[2]; v_idx[f + 1] = make_int4(base, l, c1, 1);
+  if (li == -1) {
+#pragma unroll
+    for (int q = 0; q < 3; ++q) lms[3 * static_cast<size_t>(l) + q] = p[q];
+  }
+  lm_out[i] = l;
 }
 }  // namespace hb

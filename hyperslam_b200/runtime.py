@@ -31,6 +31,7 @@ class SlideStats(C.Structure):
 
 
 SLIDE_DROP_INERTIAL = 1
+SLIDE_DROP_POSE = 2
 
 
 class Iteration(C.Structure):
@@ -55,6 +56,7 @@ EXPORTS = [
     "hb200_get_bandwidth", "hb200_set_min_bandwidth", "hb200_measure_fp64_peak", "hb200_set_reference_quirks",
     "hb200_append_knots", "hb200_append_landmarks", "hb200_append_pixel_factors", "hb200_append_inertial_factors", "hb200_slide",
     "hb200_window_sizes", "hb200_set_termination", "hb200_get_termination",
+    "hb200_append_bearing_factors", "hb200_append_manifold_factors", "hb200_append_stereo_tracks", "hb200_factor_counts",
 ]
 
 _lib = None
@@ -212,10 +214,21 @@ class Context:
         self.set_constant(w.knot_const, w.gravity_const, w.bias_const)
 
     # ---- device-side sliding-window bookkeeping ------------------------------------------------------
-    def _refresh_sizes(self):
+    def _refresh_sizes(self, counts=False):
+        """counts: also re-read the bearing / pose-prior counts (calls that can change them); Nv = pixel factors."""
         v = [C.c_int(0) for _ in range(4)]
         self._check(self.lib.hb200_window_sizes(self.h, *[C.byref(x) for x in v]))
-        self.K, self.L, self.Nv, self.Ni = (x.value for x in v)
+        self.K, self.L, self.Ni = v[0].value, v[1].value, v[3].value
+        if counts:
+            n = self.factor_counts()
+            self.Nb, self.Nm = n["bearing"], n["manifold"]
+        self.Nv = v[2].value - self.Nb
+
+    def factor_counts(self):
+        """Factors per kind: dict(pixel, bearing, inertial, manifold)."""
+        v = [C.c_int(0) for _ in range(4)]
+        self._check(self.lib.hb200_factor_counts(self.h, *[C.byref(x) for x in v]))
+        return dict(zip(("pixel", "bearing", "inertial", "manifold"), (x.value for x in v)))
 
     def append_knots(self, count=1):
         self._check(self.lib.hb200_append_knots(self.h, int(count)))
@@ -240,10 +253,39 @@ class Context:
             self._check(self.lib.hb200_append_inertial_factors(self.h, stamp.size, _d(stamp), _d(meas)))
             self._refresh_sizes()
 
-    def slide(self, lower_bound, drop_inertial=True):
+    def append_bearing_factors(self, stamp, cam, lm, bearing):
+        stamp, bearing = _f64(stamp), _f64(bearing)
+        cam, lm = np.ascontiguousarray(cam, dtype=np.int32), np.ascontiguousarray(lm, dtype=np.int32)
+        if stamp.size:
+            self._check(self.lib.hb200_append_bearing_factors(self.h, stamp.size, _d(stamp), _i(cam), _i(lm), _d(bearing)))
+            self._refresh_sizes(counts=True)
+
+    def append_manifold_factors(self, stamp, sensor, pose):
+        stamp, pose = _f64(stamp), _f64(pose)
+        sensor = np.ascontiguousarray(sensor, dtype=np.int32)
+        if stamp.size:
+            self._check(self.lib.hb200_append_manifold_factors(self.h, stamp.size, _d(stamp), _i(sensor), _d(pose)))
+            self._refresh_sizes(counts=True)
+
+    def append_stereo_tracks(self, stamp, cam0, cam1, px0, px1, landmark):
+        """process(VisualTracks): two bearing factors per track; landmark[i] == -1 triangulates and appends a new
+        landmark.  Returns every track's landmark slot (new ones take L, L+1, ... in track order)."""
+        stamp, px0, px1 = _f64(stamp), _f64(px0), _f64(px1)
+        cam0, cam1 = np.ascontiguousarray(cam0, dtype=np.int32), np.ascontiguousarray(cam1, dtype=np.int32)
+        landmark = np.ascontiguousarray(landmark, dtype=np.int32)
+        out = np.zeros(stamp.size, dtype=np.int32)
+        if stamp.size:
+            num_new = C.c_int(0)
+            self._check(self.lib.hb200_append_stereo_tracks(self.h, stamp.size, _d(stamp), _i(cam0), _i(cam1), _d(px0), _d(px1), _i(landmark),
+                                                            _i(out), C.byref(num_new)))
+            self._refresh_sizes(counts=True)
+        return out
+
+    def slide(self, lower_bound, drop_inertial=True, drop_pose=False):
         st = SlideStats()
-        self._check(self.lib.hb200_slide(self.h, C.c_double(lower_bound), SLIDE_DROP_INERTIAL if drop_inertial else 0, C.byref(st)))
-        self._refresh_sizes()
+        flags = (SLIDE_DROP_INERTIAL if drop_inertial else 0) | (SLIDE_DROP_POSE if drop_pose else 0)
+        self._check(self.lib.hb200_slide(self.h, C.c_double(lower_bound), flags, C.byref(st)))
+        self._refresh_sizes(counts=self.Nb > 0 or self.Nm > 0)
         return {n: getattr(st, n) for n, _ in SlideStats._fields_}
 
     def index_maps(self):
